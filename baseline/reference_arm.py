@@ -3,26 +3,21 @@ from __future__ import annotations
 
 import json
 import os
-import shutil
 import sys
 import time
 
+from oracle import reference
+
 HERE = os.path.dirname(os.path.abspath(__file__))
-REF_DIR = os.path.join(HERE, "_ref")
+REF_DIR = reference.REF_DIR
 SHIMS = os.path.join(HERE, "shims")
-REF_SRC = "/root/reference"
 
 
 def _ensure_ref():
-    need = ["run_vit_training.py", "utils.py"]
-    if all(os.path.exists(os.path.join(REF_DIR, f)) for f in need):
+    if reference.is_staged():
         return None
-    if not os.path.isdir(REF_SRC):
-        return f"baseline/_ref is missing and {REF_SRC} is not available to copy it from"
-    os.makedirs(REF_DIR, exist_ok=True)
-    for f in need:
-        shutil.copy(os.path.join(REF_SRC, f), os.path.join(REF_DIR, f))
-    return None
+    return ("oracle/_ref is missing: build with VIT_REFERENCE_DIR set to a checkout of the original example to "
+            "stage its script there")
 
 
 def run(args, MODELS, ClockSampler, time_steps):

@@ -5,6 +5,7 @@
     python -m torch.distributed.run --nnodes=1 --nproc-per-node 8 --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus 8 --steps 5 --warmup 3
     python bench.py --impl reference ...              # the UNMODIFIED reference script on stock PyTorch
+    python bench.py --dump-outputs DIR ...            # also write what the last timed step computed to DIR/*.npy
 
 The timed step is the body of the reference's training loop (run_vit_training.py:259-280): forward + loss, backward,
 clip_grad_norm_ on the full gradient, optimizer.step, lr_scheduler.step, zero_grad.
@@ -61,6 +62,10 @@ def parse():
     ap.add_argument("--no_e2e", action="store_true")
     ap.add_argument("--cuda_graph", type=int, default=-1,
                     help="1/0: replay the training step as one CUDA graph; -1 = auto (on for launch-bound models)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed to DIR/<name>.npy (float32): its "
+                         "loss and gradient norm, and a fixed sample of the parameters and AdamW first moments it "
+                         "left behind")
     return ap.parse_args()
 
 
@@ -154,6 +159,39 @@ def _time_steps(torch, dist, world, step_fn, steps):
     return float(ms.item())
 
 
+DUMP_SAMPLE = 1 << 20  # sampled values per array over all ranks (4 MB of float32)
+
+
+def _dump_outputs(torch, dist, world, rank, model, last, out_dir):
+    """Writes what the last training step computed as float32 .npy files: the loss and gradient norm it returned,
+    and the parameters / AdamW first moments it left behind, sampled at indices drawn from a fixed seed so that two
+    builds run with the same arguments can be compared value by value."""
+    import numpy as np
+
+    per_unit = max(1, DUMP_SAMPLE // (world * len(model.all_units)))
+    gen = torch.Generator().manual_seed(0)
+    params, moments = [], []
+    for u in model.all_units:
+        n = u.layout.shard_numel
+        idx = torch.randint(n, (min(n, per_unit),), generator=gen).to(model.device)
+        w = torch.empty(idx.numel(), dtype=torch.float32, device=model.device)
+        # the fp32 master lives split in bf16 hi + int16 lo halves: merge only the sampled entries
+        model.ops.merge_fp32(u.hi.index_select(0, idx), u.lo.index_select(0, idx), w)
+        params.append(w)
+        moments.append(u.exp_avg.index_select(0, idx))
+    out = {"loss": last["loss"], "grad_norm": last["grad_norm"], "params_sample": torch.cat(params),
+           "exp_avg_sample": torch.cat(moments)}
+    if world > 1:
+        for k in ("params_sample", "exp_avg_sample"):
+            parts = [torch.empty_like(out[k]) for _ in range(world)]
+            dist.all_gather(parts, out[k])
+            out[k] = torch.cat(parts)
+    if rank == 0:
+        os.makedirs(out_dir, exist_ok=True)
+        for k, v in out.items():
+            np.save(os.path.join(out_dir, k + ".npy"), v.detach().float().reshape(-1).cpu().numpy())
+
+
 def run_ours(args):
     import torch
     import torch.distributed as dist
@@ -197,6 +235,7 @@ def run_ours(args):
     dev_target = host_target.to(device)
     h2d_bytes = host_images.numel() * host_images.element_size() + host_target.numel() * host_target.element_size()
     last_loss = [0.0]
+    last = {}  # device tensors returned by the latest step (kept without a host sync)
 
     use_graph = args.cuda_graph == 1 or (args.cuda_graph == -1 and dim < 2048)
     graphed = None
@@ -208,12 +247,14 @@ def run_ours(args):
     def train_step(images, target):
         if graphed is not None:
             loss = graphed(images, target)
+            norm = graphed.grad_norm
         else:
             loss = model.forward_backward(images, target)
-            model.clip_grad_norm_(1.0)
+            norm = model.clip_grad_norm_(1.0)
             opt.step()
         sched.step()
         opt.zero_grad(set_to_none=True)
+        last.update(loss=loss, grad_norm=norm)
         return loss
 
     def step_e2e():
@@ -240,6 +281,8 @@ def run_ours(args):
         launches = graphed.launches_per_step * args.steps
     clocks = sampler.stop() if sampler else {}
     peak_gb = torch.cuda.max_memory_allocated() / 1e9
+    if args.dump_outputs:  # before the probes below take further optimizer steps
+        _dump_outputs(torch, dist, world, rank, model, last, args.dump_outputs)
     exposed = None
     if graphed is None:
         # Secondary metric of BASELINE.json: exposed communication per step, probed outside the timed region.
