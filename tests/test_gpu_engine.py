@@ -144,12 +144,12 @@ def test_lean_blocks_vs_recompute(heads, dim):
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("heads,dim,img", [(4, 256, 112), (2, 256, 224), (2, 320, 224), (2, 320, 336)])
-def test_flash_attention_engine_path(heads, dim, img, monkeypatch):
+def test_fused_attention_pair_matches_unfused_in_the_engine(heads, dim, img, monkeypatch):
     """Same model, same data: gradients with the flash-style attention pair (lse + fused backward kernels) must
-    match the default path (GEMMs + softmax kernels) to bf16 noise.  Covers N = 64 / 256 / 576 (the 336 px
+    match the un-fused path (GEMMs + softmax kernels, forced by replacing the plan) to bf16 noise.  Covers N = 64 / 256 / 576 (the 336 px
     long-sequence kernels), hd = 64 / 128 / 160."""
     from vit_10b_fsdp_example_b200.config import ViTConfig
-    from vit_10b_fsdp_example_b200.ops import cuda_ops as co
+    from vit_10b_fsdp_example_b200.ops import attention_plan as ap
     from vit_10b_fsdp_example_b200.parallel import FSDPViT
 
     cfg = ViTConfig(image_size=img, patch_size=14, embed_dim=dim, num_heads=heads, num_blocks=2, mlp_ratio=4.0,
@@ -159,9 +159,11 @@ def test_flash_attention_engine_path(heads, dim, img, monkeypatch):
     x = torch.randn(4, 3, img, img, generator=g).to(dev)
     y = torch.randint(0, 96, (4,), generator=g).to(dev)
     res = []
+    default_plan = ap.plan
+    assert default_plan(cfg.num_patches, cfg.head_dim).fwd_lse is not None
+    unfused = ap.AttentionPlan(None, ap.UNFUSED, None)
     for flash in (False, True):
-        monkeypatch.setattr(co, "FLASH_ATTENTION", flash)
-        monkeypatch.setattr(co, "_FLASH_ENV", "1" if flash else "0")  # force the pair on for hd = 160 too
+        monkeypatch.setattr(ap, "plan", default_plan if flash else (lambda N, hd: unfused))
         for keep in (0, 2):
             model = FSDPViT(cfg, device=dev, dtype=torch.bfloat16, seed=4, ckpt_keep_blocks=keep)
             loss = model.forward_backward(x, y).item()

@@ -1,5 +1,6 @@
-"""Attention variants at the headline shapes: un-fused (batched GEMMs + softmax kernels), one-shot fused, persistent
-fused; forward and backward.  CUDA-event timing, inputs >> L2 (qkv is 1 GB at the ViT-10B shape).
+"""Attention variants at the headline shapes: un-fused (batched GEMMs + softmax kernels), one-shot fused, long,
+persistent fused (hd = 160); forward and backward.  Every variant is launched through its own extension entry point,
+whatever ops/attention_plan.py would choose.  CUDA-event timing, inputs >> L2 (qkv is 1 GB at the ViT-10B shape).
 
     python tools/exp_attn2.py [--shapes 10b,l,336] [--json gpurun_out/attn_times.json]
 """
@@ -53,36 +54,34 @@ def main():
         res = {"shape": [B, N, H, hd]}
         flops_fwd = 4.0 * B * H * N * N * hd
         try:
+            out = torch.empty(B * N, D, dtype=qkv.dtype, device="cuda")
+            lse = torch.empty(B * H, N, device="cuda")
+            guarded("fwd_unfused_us", lambda: co.attention_fwd(qkv, B, N, H, hd, need_p=True), res)
             if N <= 256:
-                co.FUSED_ATTENTION = False
-                guarded("fwd_unfused_us", lambda: co.attention_fwd(qkv, B, N, H, hd, need_p=True), res)
-                co.FUSED_ATTENTION = True
-                co.FUSED_ATTENTION_HD160 = True
-                guarded("fwd_oneshot_us", lambda: co.attention_fwd(qkv, B, N, H, hd, need_p=False), res)
-                out, lse = co.attention_fwd_lse(qkv, B, N, H, hd)
-                if "persist_fwd" not in skip and co._C.attention_fwd_persist_supported(N, hd):
-                    o2 = torch.empty_like(out)
-                    l2 = torch.empty_like(lse)
+                guarded("fwd_oneshot_us", lambda: co._C.attention_fwd(qkv, out, lse, B, N, H, hd), res)
+                if "persist_fwd" not in skip and hd == 160 and N > 128:
+                    o2, l2 = torch.empty_like(out), torch.empty_like(lse)
                     guarded("fwd_persist_us", lambda: co._C.attention_fwd_persist(qkv, o2, l2, B, N, H, hd), res)
                     res["fwd_persist_max_err_vs_oneshot"] = float((o2.float() - out.float()).abs().max())
             else:
-                co.FLASH_LONG = True
-                guarded("fwd_unfused_us", lambda: co.attention_fwd(qkv, B, N, H, hd, need_p=True), res)
-                guarded("fwd_long_us", lambda: co.attention_fwd_lse(qkv, B, N, H, hd), res)
-                out, lse = co.attention_fwd_lse(qkv, B, N, H, hd)
-            _, p = (co.FUSED_ATTENTION and N <= 256 and (setattr(co, "FUSED_ATTENTION", False) or True)) and co.attention_fwd(qkv, B, N, H, hd, need_p=True) or co.attention_fwd(qkv, B, N, H, hd, need_p=True)
+                guarded("fwd_long_us", lambda: co._C.attention_fwd_long(qkv, out, lse, B, N, H, hd), res)
+            _, p = co.attention_fwd(qkv, B, N, H, hd, need_p=True)
             guarded("bwd_unfused_us", lambda: co.attention_bwd(dout, qkv, p, B, N, H, hd, want_colsum=True), res)
             guarded("probs_remat_us", lambda: co.attention_probs(qkv, B, N, H, hd), res)
             del p
-            co.ATTN_PERSIST = False
-            guarded("bwd_fused_us", lambda: co.attention_bwd_lse(dout, qkv, out, lse, B, N, H, hd, want_colsum=True), res)
-            if "persist_bwd" not in skip:
-                ref = co.attention_bwd_lse(dout, qkv, out, lse, B, N, H, hd)
-                co.ATTN_PERSIST = True
-                guarded("bwd_persist_us", lambda: co.attention_bwd_lse(dout, qkv, out, lse, B, N, H, hd, want_colsum=True), res)
-                got = co.attention_bwd_lse(dout, qkv, out, lse, B, N, H, hd)
-                res["bwd_persist_max_err_vs_fused"] = float((got.float() - ref.float()).abs().max())
-                co.ATTN_PERSIST = False
+
+            def bwd(persist):  # delta kernel + dK/dV + dQ kernels + qkv bias gradient, as attention_bwd_lse runs them
+                dqkv = torch.empty(B * N, 3 * D, dtype=qkv.dtype, device="cuda")
+                delta = torch.empty(2 if persist else 1, B * H, N, device="cuda")
+                cs = torch.zeros(3 * D, device="cuda") if persist else None
+                co._C.attention_bwd(qkv, dout, out, lse, delta, dqkv, cs, B, N, H, hd, persist)
+                return dqkv, (cs if persist else co.colsum(dqkv))
+
+            guarded("bwd_oneshot_us", lambda: bwd(False), res)
+            if "persist_bwd" not in skip and hd == 160 and N % 4 == 0:
+                ref = bwd(False)[0]
+                guarded("bwd_persist_us", lambda: bwd(True), res)
+                res["bwd_persist_max_err_vs_oneshot"] = float((bwd(True)[0].float() - ref.float()).abs().max())
         except Exception as ex:
             res["error"] = f"{type(ex).__name__}: {str(ex)[:200]}"
             allres[key] = res

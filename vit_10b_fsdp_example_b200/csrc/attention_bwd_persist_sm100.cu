@@ -15,7 +15,7 @@
 //     qkv bias gradient (column sums of dq / dk / dv) is reduced from that staging tile instead of re-reading the
 //     1 GB dqkv tensor with a separate kernel;
 //   * key / query masks are compiled out when N is a multiple of 128.
-// Default for hd > 128 (validated on B200: tests/test_gpu_attention.py::test_persistent_attention_backward).
+// Instantiated for hd = 160 only; chosen there when N % 4 == 0 (ops/attention_plan.py).
 #include <cuda.h>
 #include <cuda_runtime.h>
 #include <cuda_bf16.h>
@@ -553,13 +553,7 @@ template <int HD>
 void run_bwd_persist(const GemmOperand& q, const GemmOperand& k, const GemmOperand& v, const GemmOperand& dO,
                      BwdPParams p, __nv_bfloat16* dqkv, float* colsum, cudaStream_t stream) {
     // dq / dk / dv slices of dqkv viewed as [B][H][N rows, hd columns]: what the epilogue's TMA stores address
-    GemmOperand oq, ok, ov;
-    oq.ptr = dqkv, ok.ptr = dqkv + p.D, ov.ptr = dqkv + 2 * p.D;
-    for (GemmOperand* o : {&oq, &ok, &ov}) {
-        o->ld = p.ld_out;
-        o->nb_inner = p.H, o->stride_b_inner = HD;
-        o->nb_outer = p.B, o->stride_b_outer = static_cast<int64_t>(p.N) * p.ld_out;
-    }
+    const auto [oq, ok, ov] = qkv_operands(dqkv, p.ld_out, p.B, p.N, p.H, HD);
     const bool mask = p.N % 128 != 0;
     p.out1 = dqkv + p.D, p.out2 = dqkv + 2 * p.D;
     p.colsum1 = colsum != nullptr ? colsum + p.D : nullptr;
@@ -587,14 +581,12 @@ void attention_bwd_set_trace(long long* buf, int tiles, int role) {
 void attention_bwd_persist_core(const __nv_bfloat16* qkv, int64_t ld_qkv, const __nv_bfloat16* dout, int64_t ld_do,
                                 const float* lse, const float* delta, __nv_bfloat16* dqkv, float* colsum, int B, int N,
                                 int H, int hd, cudaStream_t stream) {
+    // instantiated for hd = 160 only: where two one-shot CTAs fit an SM (hd <= 128) those win; the per-row
+    // statistics are bulk-copied in 16-byte units
+    if (hd != 160 || N % 4 != 0) throw std::runtime_error("attention_bwd_persist: unsupported (N, head_dim)");
     const int D = H * hd;
-    GemmOperand q, k, v, dO;
-    q.ptr = qkv, k.ptr = qkv + D, v.ptr = qkv + 2 * D, dO.ptr = dout;
-    for (GemmOperand* o : {&q, &k, &v, &dO}) {
-        o->ld = (o == &dO) ? ld_do : ld_qkv;
-        o->nb_inner = H, o->stride_b_inner = hd;
-        o->nb_outer = B, o->stride_b_outer = static_cast<int64_t>(N) * o->ld;
-    }
+    const auto [q, k, v] = qkv_operands(qkv, ld_qkv, B, N, H, hd);
+    const GemmOperand dO = head_operand(dout, ld_do, B, N, H, hd);
     BwdPParams p;
     p.N = N, p.H = H, p.B = B, p.D = D;
     p.nblk = (N + 127) / 128;
@@ -606,9 +598,7 @@ void attention_bwd_persist_core(const __nv_bfloat16* qkv, int64_t ld_qkv, const 
     p.colsum1 = p.colsum2 = nullptr;
     p.trace = g_bwd_trace, p.trace_tiles = g_bwd_trace_tiles;
     p.ld_out = 3 * static_cast<int64_t>(D);
-    if (hd == 64) run_bwd_persist<64>(q, k, v, dO, p, dqkv, colsum, stream);
-    else if (hd == 128) run_bwd_persist<128>(q, k, v, dO, p, dqkv, colsum, stream);
-    else run_bwd_persist<160>(q, k, v, dO, p, dqkv, colsum, stream);
+    run_bwd_persist<160>(q, k, v, dO, p, dqkv, colsum, stream);
 }
 
 }  // namespace b200

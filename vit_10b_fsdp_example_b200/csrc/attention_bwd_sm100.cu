@@ -51,17 +51,6 @@ struct AttnBwdParams {
     int64_t ld_out;       // 3 * D
 };
 
-// generic shared-memory matrix descriptor (field layout in ptx.cuh); layout: 2 = SWIZZLE_128B, 4 = SWIZZLE_64B
-__device__ __forceinline__ uint64_t smem_desc(uint32_t addr, uint32_t lbo, uint32_t sbo, uint32_t layout) {
-    uint64_t d = 0;
-    d |= static_cast<uint64_t>((addr >> 4) & 0x3FFF);
-    d |= static_cast<uint64_t>((lbo >> 4) & 0x3FFF) << 16;
-    d |= static_cast<uint64_t>((sbo >> 4) & 0x3FFF) << 32;
-    d |= static_cast<uint64_t>(1) << 46;
-    d |= static_cast<uint64_t>(layout) << 61;
-    return d;
-}
-
 template <int HD, bool kT>
 struct BwdCfg {
     static constexpr int W = (HD % 64 == 0) ? 64 : 32;        // hd columns per swizzle atom
@@ -190,8 +179,8 @@ __global__ void __launch_bounds__(kBwdThreads) attn_bwd_sm100_kernel(const __gri
 #pragma unroll
                 for (int k = 0; k < HD / 16; ++k) {
                     const int atom = (k * 16) / W, within = (k * 16) % W;
-                    const uint64_t da = smem_desc(smem_u32(sx) + atom * (128 * kRowBytes) + within * 2, 0, kSbo, kLayout);
-                    const uint64_t db = smem_desc(smem_u32(sy) + atom * (kTileC * kRowBytes) + within * 2, 0, kSbo, kLayout);
+                    const uint64_t da = make_smem_desc(smem_u32(sx) + atom * (128 * kRowBytes) + within * 2, 0, kSbo, kLayout);
+                    const uint64_t db = make_smem_desc(smem_u32(sy) + atom * (kTileC * kRowBytes) + within * 2, 0, kSbo, kLayout);
                     umma_bf16<1>(tmem_d, da, db, idesc_t, k > 0 ? 1u : 0u);
                 }
             };
@@ -199,9 +188,9 @@ __global__ void __launch_bounds__(kBwdThreads) attn_bwd_sm100_kernel(const __gri
             auto issue_acc = [&](uint32_t tmem_d, const uint8_t* se, const uint8_t* sy, bool accumulate) {
 #pragma unroll
                 for (int k = 0; k < kTileC / 16; ++k) {
-                    const uint64_t da = smem_desc(smem_u32(se) + k * 32, 0, 1024, 2u);
+                    const uint64_t da = make_smem_desc(smem_u32(se) + k * 32, 0, 1024, 2u);
                     // MN-major B: 8-row groups are 8*rowbytes apart (SBO), hd atoms are 64*rowbytes apart (LBO)
-                    const uint64_t db = smem_desc(smem_u32(sy) + k * 16 * kRowBytes, kTileC * kRowBytes, kSbo, kLayout);
+                    const uint64_t db = make_smem_desc(smem_u32(sy) + k * 16 * kRowBytes, kTileC * kRowBytes, kSbo, kLayout);
                     umma_bf16<1>(tmem_d, da, db, idesc_a, (accumulate || k > 0) ? 1u : 0u);
                 }
             };
@@ -495,8 +484,8 @@ __global__ void __launch_bounds__(kBwdThreads) attn_fwd_long_sm100_kernel(const 
 #pragma unroll
                 for (int k = 0; k < HD / 16; ++k) {
                     const int atom = (k * 16) / W, within = (k * 16) % W;
-                    const uint64_t da = smem_desc(smem_u32(sQ) + atom * (128 * kRowBytes) + within * 2, 0, kSbo, kLayout);
-                    const uint64_t db = smem_desc(smem_u32(sy) + atom * (kTileC * kRowBytes) + within * 2, 0, kSbo, kLayout);
+                    const uint64_t da = make_smem_desc(smem_u32(sQ) + atom * (128 * kRowBytes) + within * 2, 0, kSbo, kLayout);
+                    const uint64_t db = make_smem_desc(smem_u32(sy) + atom * (kTileC * kRowBytes) + within * 2, 0, kSbo, kLayout);
                     umma_bf16<1>(tmem_d, da, db, idesc_t, k > 0 ? 1u : 0u);
                 }
             };
@@ -525,8 +514,8 @@ __global__ void __launch_bounds__(kBwdThreads) attn_fwd_long_sm100_kernel(const 
                     tc_fence_after();
 #pragma unroll
                     for (int k = 0; k < kTileC / 16; ++k) {
-                        const uint64_t da = smem_desc(smem_u32(sE) + k * 32, 0, 1024, 2u);
-                        const uint64_t db = smem_desc(smem_u32(yv) + k * 16 * kRowBytes, kTileC * kRowBytes, kSbo, kLayout);
+                        const uint64_t da = make_smem_desc(smem_u32(sE) + k * 32, 0, 1024, 2u);
+                        const uint64_t db = make_smem_desc(smem_u32(yv) + k * 16 * kRowBytes, kTileC * kRowBytes, kSbo, kLayout);
                         umma_bf16<1>(tmem_base + C::kColAcc, da, db, idesc_a, (i > 0 || k > 0) ? 1u : 0u);
                     }
                     umma_commit<1>(e_empty);
@@ -722,32 +711,25 @@ void launch_fwd_long(const GemmOperand& q, const GemmOperand& k, const GemmOpera
         throw std::runtime_error(std::string("attention fwd-long launch: ") + cudaGetErrorString(err));
 }
 
-}  // namespace
-
 bool attention_fwd_long_supported(int N, int hd) { return N % 2 == 0 && (hd == 64 || hd == 128 || hd == 160); }
+
+bool attention_bwd_supported(int N, int hd) {
+    return N <= kMaxSeq && N % 2 == 0 && (hd == 64 || hd == 128 || hd == 160);
+}
+
+}  // namespace
 
 void attention_fwd_long(const __nv_bfloat16* qkv, int64_t ld_qkv, __nv_bfloat16* out, float* lse, int B, int N, int H,
                         int hd, cudaStream_t stream) {
     if (!attention_fwd_long_supported(N, hd)) throw std::runtime_error("attention_fwd_long: unsupported (N, head_dim)");
-    const int D = H * hd;
-    GemmOperand q, k, v;
-    q.ptr = qkv, k.ptr = qkv + D, v.ptr = qkv + 2 * D;
-    for (GemmOperand* o : {&q, &k, &v}) {
-        o->ld = ld_qkv;
-        o->nb_inner = H, o->stride_b_inner = hd;
-        o->nb_outer = B, o->stride_b_outer = static_cast<int64_t>(N) * ld_qkv;
-    }
+    const auto [q, k, v] = qkv_operands(qkv, ld_qkv, B, N, H, hd);
     AttnFwdLongParams p;
-    p.N = N, p.H = H, p.B = B, p.D = D;
+    p.N = N, p.H = H, p.B = B, p.D = H * hd;
     p.scale_log2 = 1.4426950408889634f / sqrtf(static_cast<float>(hd));
     p.out = out, p.lse = lse;
     if (hd == 64) launch_fwd_long<64>(q, k, v, p, stream);
     else if (hd == 128) launch_fwd_long<128>(q, k, v, p, stream);
     else launch_fwd_long<160>(q, k, v, p, stream);
-}
-
-bool attention_bwd_supported(int N, int hd) {
-    return N <= kMaxSeq && N % 2 == 0 && (hd == 64 || hd == 128 || hd == 160);
 }
 
 void attention_bwd(const __nv_bfloat16* qkv, int64_t ld_qkv, const __nv_bfloat16* dout, int64_t ld_do,
@@ -770,13 +752,8 @@ void attention_bwd(const __nv_bfloat16* qkv, int64_t ld_qkv, const __nv_bfloat16
         return;
     }
     if (colsum != nullptr) throw std::runtime_error("attention_bwd: fused column sums need the persistent kernels");
-    GemmOperand q, k, v, dO;
-    q.ptr = qkv, k.ptr = qkv + D, v.ptr = qkv + 2 * D, dO.ptr = dout;
-    for (GemmOperand* o : {&q, &k, &v, &dO}) {
-        o->ld = (o == &dO) ? ld_do : ld_qkv;
-        o->nb_inner = H, o->stride_b_inner = hd;
-        o->nb_outer = B, o->stride_b_outer = static_cast<int64_t>(N) * o->ld;
-    }
+    const auto [q, k, v] = qkv_operands(qkv, ld_qkv, B, N, H, hd);
+    const GemmOperand dO = head_operand(dout, ld_do, B, N, H, hd);
     AttnBwdParams p;
     p.N = N, p.H = H, p.B = B, p.D = D;
     p.scale = 1.0f / sqrtf(static_cast<float>(hd));

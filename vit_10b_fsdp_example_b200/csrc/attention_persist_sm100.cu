@@ -1,4 +1,4 @@
-// Persistent, software-pipelined attention forward for sm_100a (128 < N <= 256 tokens, head dim 64 / 128 / 160).
+// Persistent, software-pipelined attention forward for sm_100a (128 < N <= 256 tokens, head dim 160).
 //
 // The one-shot kernel in attention_sm100.cu runs load -> S MMA -> softmax -> PV MMA -> store strictly in sequence and
 // only one CTA fits an SM at hd = 160 (200 KB of shared memory), so nothing hides its loads (ncu: tensor pipe 9 %,
@@ -384,11 +384,10 @@ void launch_persist(const GemmOperand& q, const GemmOperand& k, const GemmOperan
         throw std::runtime_error(std::string("attention persist launch: ") + cudaGetErrorString(err));
 }
 
-}  // namespace
+// Instantiated for hd = 160 only: where two one-shot CTAs fit an SM (hd <= 128) those win.
+bool attention_fwd_persist_supported(int N, int hd) { return N > 128 && N <= 256 && N % 2 == 0 && hd == 160; }
 
-bool attention_fwd_persist_supported(int N, int hd) {
-    return N > 128 && N <= 256 && N % 2 == 0 && (hd == 64 || hd == 128 || hd == 160);
-}
+}  // namespace
 
 // Optional in-kernel timeline (SURVEY 5.1): clock64 stamps of CTA 0's producer / MMA / softmax roles, 16 per work item.
 static long long* g_trace = nullptr;
@@ -400,13 +399,7 @@ void attention_fwd_persist(const __nv_bfloat16* qkv, int64_t ld_qkv, __nv_bfloat
     if (!attention_fwd_persist_supported(N, hd))
         throw std::runtime_error("attention_fwd_persist: unsupported (N, head_dim)");
     const int D = H * hd;
-    GemmOperand q, k, v;
-    q.ptr = qkv, k.ptr = qkv + D, v.ptr = qkv + 2 * D;
-    for (GemmOperand* o : {&q, &k, &v}) {
-        o->ld = ld_qkv;
-        o->nb_inner = H, o->stride_b_inner = hd;
-        o->nb_outer = B, o->stride_b_outer = static_cast<int64_t>(N) * ld_qkv;
-    }
+    const auto [q, k, v] = qkv_operands(qkv, ld_qkv, B, N, H, hd);
     PersistParams p;
     p.N = N, p.H = H, p.B = B, p.D = D;
     p.nq = (N + 127) / 128;
@@ -416,18 +409,9 @@ void attention_fwd_persist(const __nv_bfloat16* qkv, int64_t ld_qkv, __nv_bfloat
     p.scale_log2 = p.scale * 1.4426950408889634f;
     p.out = out, p.lse = lse;
     p.trace = g_trace, p.trace_items = g_trace_items;
-    GemmOperand o;  // out viewed as [B][H][N rows, hd columns]: what the epilogue's TMA stores address
-    o.ptr = out, o.ld = D;
-    o.nb_inner = H, o.stride_b_inner = hd;
-    o.nb_outer = B, o.stride_b_outer = static_cast<int64_t>(N) * D;
-    const bool mask = N % kVT != 0;  // key columns beyond N exist only in a ragged last tile
-#define B200_PERSIST(HDV)                                                  \
-    if (mask) launch_persist<HDV, true>(q, k, v, o, p, stream);            \
-    else launch_persist<HDV, false>(q, k, v, o, p, stream)
-    if (hd == 64) { B200_PERSIST(64); }
-    else if (hd == 128) { B200_PERSIST(128); }
-    else { B200_PERSIST(160); }
-#undef B200_PERSIST
+    const GemmOperand o = head_operand(out, D, B, N, H, hd);  // what the epilogue's TMA stores address
+    if (N % kVT != 0) launch_persist<160, true>(q, k, v, o, p, stream);  // key columns beyond N: ragged last tile
+    else launch_persist<160, false>(q, k, v, o, p, stream);
 }
 
 }  // namespace b200

@@ -8,10 +8,9 @@
 //             O re-uses the TMEM columns of S, so a CTA needs only NK columns and two CTAs fit an SM for hd=64.
 //   softmax : one thread per query row straight out of TMEM (tcgen05.ld), exp2 with the scale folded in,
 //             two passes (max, then exp/sum), un-normalised P to smem, 1/sum applied to O in the epilogue.
-//   outputs : O [tokens, D] bf16, log-sum-exp per row (fp32), optionally the normalised probabilities P
-//             (needed by the un-fused backward).
+//   outputs : O [tokens, D] bf16, optionally the log-sum-exp per row (fp32) for the fused backward.
 //
-// Scores never reach HBM (unless P is requested).  Replaces timm Attention's materialised [B,H,N,N] softmax
+// Scores never reach HBM.  Replaces timm Attention's materialised [B,H,N,N] softmax
 // (reference run_vit_training.py:134 -> timm Block -> Attention).
 #include <cuda.h>
 #include <cuda_runtime.h>
@@ -40,20 +39,7 @@ struct AttnParams {
     float scale;       // hd^-1/2
     __nv_bfloat16* out;  // [B*N, D]
     float* lse;          // [B*H, N] or null
-    __nv_bfloat16* p;    // [B*H, N, ldp] or null
-    int64_t ldp;
 };
-
-// generic shared-memory matrix descriptor (see ptx.cuh for the field layout); layout: 2 = SW128, 4 = SW64
-__device__ __forceinline__ uint64_t smem_desc(uint32_t addr, uint32_t lbo, uint32_t sbo, uint32_t layout) {
-    uint64_t d = 0;
-    d |= static_cast<uint64_t>((addr >> 4) & 0x3FFF);
-    d |= static_cast<uint64_t>((lbo >> 4) & 0x3FFF) << 16;
-    d |= static_cast<uint64_t>((sbo >> 4) & 0x3FFF) << 32;
-    d |= static_cast<uint64_t>(1) << 46;
-    d |= static_cast<uint64_t>(layout) << 61;
-    return d;
-}
 
 template <int HD, int NK>
 __global__ void __launch_bounds__(kAttnThreads) attn_fwd_sm100_kernel(const __grid_constant__ CUtensorMap tmap_q,
@@ -127,8 +113,8 @@ __global__ void __launch_bounds__(kAttnThreads) attn_fwd_sm100_kernel(const __gr
 #pragma unroll
             for (int k = 0; k < HD / 16; ++k) {
                 const int atom = (k * 16) / W, within = (k * 16) % W;
-                const uint64_t da = smem_desc(smem_u32(sQ) + atom * (128 * kRowBytes) + within * 2, 0, kSbo, kLayout);
-                const uint64_t db = smem_desc(smem_u32(sK) + atom * (NK * kRowBytes) + within * 2, 0, kSbo, kLayout);
+                const uint64_t da = make_smem_desc(smem_u32(sQ) + atom * (128 * kRowBytes) + within * 2, 0, kSbo, kLayout);
+                const uint64_t db = make_smem_desc(smem_u32(sK) + atom * (NK * kRowBytes) + within * 2, 0, kSbo, kLayout);
                 umma_bf16<1>(tmem_base, da, db, idesc_s, k > 0 ? 1u : 0u);
             }
             umma_commit<1>(bar_s);
@@ -141,9 +127,9 @@ __global__ void __launch_bounds__(kAttnThreads) attn_fwd_sm100_kernel(const __gr
 #pragma unroll
             for (int k = 0; k < NK / 16; ++k) {
                 const int patom = (k * 16) / 64, pwithin = (k * 16) % 64;
-                const uint64_t da = smem_desc(smem_u32(sK) + patom * (128 * 128) + pwithin * 2, 0, 1024, 2u);
+                const uint64_t da = make_smem_desc(smem_u32(sK) + patom * (128 * 128) + pwithin * 2, 0, 1024, 2u);
                 // MN-major: 8-key groups are 8*rowbytes apart (SBO), hd atoms are NK*rowbytes apart (LBO)
-                const uint64_t db = smem_desc(smem_u32(sV) + k * 16 * kRowBytes, NK * kRowBytes, kSbo, kLayout);
+                const uint64_t db = make_smem_desc(smem_u32(sV) + k * 16 * kRowBytes, NK * kRowBytes, kSbo, kLayout);
                 umma_bf16<1>(tmem_base, da, db, idesc_o, k > 0 ? 1u : 0u);
             }
             umma_commit<1>(bar_o);
@@ -199,24 +185,6 @@ __global__ void __launch_bounds__(kAttnThreads) attn_fwd_sm100_kernel(const __gr
 
         const int64_t bh = static_cast<int64_t>(b) * p.H + h;
         if (p.lse != nullptr && row_ok) p.lse[bh * p.N + q] = mx * p.scale + __logf(sum);
-        if (p.p != nullptr && row_ok) {
-            // normalised probabilities for the un-fused backward: re-read this row's bf16 P from smem
-            __nv_bfloat16* dst = p.p + (bh * p.N + q) * p.ldp;
-            for (int col = 0; col < p.N; col += 8) {
-                const uint32_t atom = col >> 6, chunk = (col & 63) >> 3;
-                const uint4 raw = *reinterpret_cast<const uint4*>(sK + r * 128 + atom * (128 * 128) + ((chunk ^ (r & 7)) << 4));
-                const uint32_t w[4] = {raw.x, raw.y, raw.z, raw.w};
-                uint32_t o[4];
-#pragma unroll
-                for (int t = 0; t < 4; ++t) o[t] = pack_bf16x2(bf16_lo(w[t]) * inv, bf16_hi(w[t]) * inv);
-                if (col + 8 <= p.N) {
-                    *reinterpret_cast<uint4*>(dst + col) = make_uint4(o[0], o[1], o[2], o[3]);
-                } else {
-                    for (int t = 0; t < p.N - col; ++t)
-                        dst[col + t] = __float2bfloat16((t & 1) ? bf16_hi(o[t >> 1]) : bf16_lo(o[t >> 1]));
-                }
-            }
-        }
 
         // ---- epilogue: O / sum -> bf16 -> out[token, h*hd + :] ----
         mbar_wait(bar_o, 0);
@@ -269,26 +237,19 @@ void launch_attn(const GemmOperand& q, const GemmOperand& k, const GemmOperand& 
     if (err != cudaSuccess) throw std::runtime_error(std::string("attention launch: ") + cudaGetErrorString(err));
 }
 
-}  // namespace
-
 bool attention_fwd_supported(int N, int hd) { return N <= 256 && (hd == 64 || hd == 128 || hd == 160) && N % 2 == 0; }
 
-void attention_fwd(const __nv_bfloat16* qkv, int64_t ld_qkv, __nv_bfloat16* out, float* lse, __nv_bfloat16* probs,
-                   int64_t ldp, int B, int N, int H, int hd, cudaStream_t stream) {
+}  // namespace
+
+void attention_fwd(const __nv_bfloat16* qkv, int64_t ld_qkv, __nv_bfloat16* out, float* lse, int B, int N, int H,
+                   int hd, cudaStream_t stream) {
     if (!attention_fwd_supported(N, hd)) throw std::runtime_error("attention_fwd: unsupported (N, head_dim)");
-    const int D = H * hd;
-    GemmOperand q, k, v;
-    q.ptr = qkv, k.ptr = qkv + D, v.ptr = qkv + 2 * D;
-    for (GemmOperand* o : {&q, &k, &v}) {
-        o->ld = ld_qkv;
-        o->nb_inner = H, o->stride_b_inner = hd;
-        o->nb_outer = B, o->stride_b_outer = static_cast<int64_t>(N) * ld_qkv;
-    }
+    const auto [q, k, v] = qkv_operands(qkv, ld_qkv, B, N, H, hd);
     AttnParams p;
-    p.N = N, p.H = H, p.B = B, p.D = D;
+    p.N = N, p.H = H, p.B = B, p.D = H * hd;
     p.scale = 1.0f / sqrtf(static_cast<float>(hd));
     p.scale_log2 = p.scale * 1.4426950408889634f;
-    p.out = out, p.lse = lse, p.p = probs, p.ldp = ldp;
+    p.out = out, p.lse = lse;
     const bool small = N <= 128;  // keys padded to 128 instead of 256 (needs hd <= 128: O re-uses S's TMEM columns)
     if (hd == 64) {
         if (small) launch_attn<64, 128>(q, k, v, p, stream);

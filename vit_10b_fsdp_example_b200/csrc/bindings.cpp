@@ -99,13 +99,10 @@ void softmax_bwd(Tensor dp, Tensor p, int64_t rows, int64_t n, int64_t ld, doubl
     b200::softmax_bwd(bf16_mut(dp), bf16_ptr(p), rows, (int)n, ld, (float)scale, cur_stream());
 }
 
-bool attention_fwd_supported(int64_t N, int64_t hd) { return b200::attention_fwd_supported((int)N, (int)hd); }
-
-void attention_fwd(Tensor qkv, Tensor out, OptT lse, OptT probs, int64_t B, int64_t N, int64_t H, int64_t hd) {
+void attention_fwd(Tensor qkv, Tensor out, OptT lse, int64_t B, int64_t N, int64_t H, int64_t hd) {
     c10::cuda::CUDAGuard guard(qkv.device());
     TORCH_CHECK(qkv.dim() == 2 && qkv.stride(1) == 1 && out.is_contiguous(), "attention_fwd: bad layouts");
-    b200::attention_fwd(bf16_ptr(qkv), qkv.stride(0), bf16_mut(out), lse.has_value() ? f32_ptr(*lse) : nullptr,
-                        probs.has_value() ? bf16_mut(*probs) : nullptr, probs.has_value() ? probs->size(2) : 0, (int)B,
+    b200::attention_fwd(bf16_ptr(qkv), qkv.stride(0), bf16_mut(out), lse.has_value() ? f32_ptr(*lse) : nullptr, (int)B,
                         (int)N, (int)H, (int)hd, cur_stream());
 }
 
@@ -118,13 +115,6 @@ void attention_fwd_long(Tensor qkv, Tensor out, Tensor lse, int64_t B, int64_t N
                              cur_stream());
 }
 
-bool attention_fwd_persist_supported(int64_t N, int64_t hd) {
-    return b200::attention_fwd_persist_supported((int)N, (int)hd);
-}
-
-bool attention_fwd_long_supported(int64_t N, int64_t hd) {
-    return b200::attention_fwd_long_supported((int)N, (int)hd);
-}
 void attention_set_trace(OptT buf) {
     if (!buf.has_value()) {
         b200::attention_set_trace(nullptr, 0);
@@ -147,8 +137,6 @@ void attention_fwd_persist(Tensor qkv, Tensor out, OptT lse, int64_t B, int64_t 
     b200::attention_fwd_persist(bf16_ptr(qkv), qkv.stride(0), bf16_mut(out), lse.has_value() ? f32_ptr(*lse) : nullptr,
                                 (int)B, (int)N, (int)H, (int)hd, cur_stream());
 }
-
-bool attention_bwd_supported(int64_t N, int64_t hd) { return b200::attention_bwd_supported((int)N, (int)hd); }
 
 void attention_bwd(Tensor qkv, Tensor dout, Tensor out, Tensor lse, Tensor delta, Tensor dqkv, OptT colsum, int64_t B,
                    int64_t N, int64_t H, int64_t hd, bool persist) {
@@ -361,15 +349,11 @@ PYBIND11_MODULE(TORCH_EXTENSION_NAME, m) {
     m.def("softmax_fwd", &softmax_fwd);
     m.def("softmax_bwd", &softmax_bwd);
     m.def("attention_fwd", &attention_fwd);
-    m.def("attention_fwd_supported", &attention_fwd_supported);
     m.def("attention_fwd_long", &attention_fwd_long);
-    m.def("attention_fwd_long_supported", &attention_fwd_long_supported);
     m.def("attention_fwd_persist", &attention_fwd_persist);
     m.def("attention_set_trace", &attention_set_trace);
     m.def("attention_bwd_set_trace", &attention_bwd_set_trace);
-    m.def("attention_fwd_persist_supported", &attention_fwd_persist_supported);
     m.def("attention_bwd", &attention_bwd);
-    m.def("attention_bwd_supported", &attention_bwd_supported);
     m.def("cross_entropy", &cross_entropy);
     m.def("im2col", &im2col);
     m.def("gelu_fwd", &gelu_fwd);

@@ -6,8 +6,8 @@ Every function launches hand-written kernels from ``_C.so``:
     forward (NT), dgrad (NN) and wgrad (TN) run on the same kernel via K-major / MN-major descriptors.
   * attention core: fused tcgen05 forward (keeps the row log-sum-exp) + fused backward kernels that read q/k/v in
     place from the packed qkv buffer through 4-D TMA tensor maps; scores never reach HBM.  The un-fused path (batched
-    tcgen05 GEMMs + softmax / softmax-backward kernels with materialised P) remains for attention dropout and
-    B200_FUSED_ATTN_BWD=0.
+    tcgen05 GEMMs + softmax / softmax-backward kernels with materialised P) serves attention dropout and the shapes
+    the fused kernels do not cover.  Which kernel runs for a shape is decided in one place: ``attention_plan.plan``.
   * LayerNorm fwd/bwd, cross-entropy, im2col, column sums, sum of squares, fused AdamW.
 
 What each group replaces in the reference (all of it reached through timm / torch_xla there):
@@ -27,7 +27,8 @@ from typing import Optional
 
 import torch
 
-from . import native
+from . import attention_plan, native
+from .attention_plan import LONG, ONESHOT, PERSIST
 
 NAME = "sm100"
 
@@ -211,21 +212,6 @@ def colsum(x):
 # ------------------------------------------------------------------------------------------------
 # Attention core
 # ------------------------------------------------------------------------------------------------
-FUSED_ATTENTION = _os.environ.get("B200_FUSED_ATTN", "1") != "0"
-FUSED_ATTENTION_HD160 = _os.environ.get("B200_FUSED_ATTN_HD160", "0") == "1"
-
-
-# Persistent, software-pipelined kernels (csrc/attention_persist_sm100.cu, attention_bwd_persist_sm100.cu): one CTA per
-# SM loops over work items.  They win where only one CTA fits an SM (hd = 160, round-2 kernels: forward 311 vs 763 us
-# one-shot, backward 1352 vs 1814 us) and lose where two fit (hd = 64: 254 vs 159 us), hence the per-shape default below.
-_PERSIST_ENV = _os.environ.get("B200_ATTN_PERSIST", "")
-ATTN_PERSIST = _PERSIST_ENV == "1"
-
-
-def _persist(hd: int) -> bool:
-    return ATTN_PERSIST or (_PERSIST_ENV != "0" and hd > 128)
-
-
 def dropout(x, p: float, key: int):
     """Philox-keyed dropout kernel (csrc/elementwise.cu): the mask is a function of (key, position), never stored."""
     xc = x.contiguous()
@@ -248,95 +234,54 @@ def mean_pool_bwd(dpooled, B: int, N: int):
 
 
 def attention_fwd(qkv, B: int, N: int, H: int, hd: int, drop=None, need_p: bool = True):
-    """Returns (out [B*N, D], P).  P = softmax probabilities [B*H, N, ldp] for the backward, or None when
-    need_p=False and the fused kernel ran (scores never reach HBM then).
+    """Returns (out [B*N, D], P).  P = softmax probabilities [B*H, N, ldp] for the backward, or None when a fused
+    kernel ran (scores never reach HBM then); need_p=True always takes the un-fused path.
     drop = (p, key): attention dropout.  The probabilities are materialised (un-fused path), the dropped copy that
     feeds P V comes from the Philox dropout kernel; the returned P is the un-dropped one (backward regenerates the mask)."""
     D = H * hd
-    ldp = _pad8(N)
-    if drop is not None:
-        p = attention_probs(qkv, B, N, H, hd)
-        pd = dropout(p, drop[0], drop[1])
-        out = torch.empty(B * N, D, dtype=qkv.dtype, device=qkv.device)
-        ld3 = qkv.stride(0)
-        gemm_raw(pd, ldp, 0, qkv[:, 2 * D:], ld3, 1, out, D, N, hd, N,
-                 batch=(H, B, N * ldp, H * N * ldp, hd, N * ld3, hd, N * D))
-        return out, p
-    if _persist(hd) and FUSED_ATTENTION and not need_p and _C.attention_fwd_persist_supported(N, hd):
-        out = torch.empty(B * N, D, dtype=qkv.dtype, device=qkv.device)
+    out = torch.empty(B * N, D, dtype=qkv.dtype, device=qkv.device)
+    kernel = None if (need_p or drop is not None) else attention_plan.plan(N, hd).fwd
+    if kernel == PERSIST:
         _C.attention_fwd_persist(qkv, out, None, B, N, H, hd)
         return out, None
-    # hd <= 128: two CTAs fit an SM and the one-shot fused kernel is ~1.8x faster than GEMM+softmax+GEMM (ViT-L: 159 vs
-    # 279 us).  hd = 160 (ViT-10B) needs 200 KB of smem -> one CTA per SM: that shape runs the persistent kernel above
-    # (311 us); the one-shot kernel (764 us) loses to the batched-GEMM path (664 us) there and is only used when forced.
-    if FUSED_ATTENTION and _C.attention_fwd_supported(N, hd) and (hd <= 128 or FUSED_ATTENTION_HD160):
-        # one fused tcgen05 kernel per (image, head, 128-query block): S and P live in TMEM / shared memory
-        out = torch.empty(B * N, D, dtype=qkv.dtype, device=qkv.device)
-        p = None
-        if need_p:
-            p = torch.empty(B * H, N, ldp, dtype=qkv.dtype, device=qkv.device)
-            if ldp != N:
-                p[:, :, N:].zero_()
-        _C.attention_fwd(qkv, out, None, p, B, N, H, hd)
-        return out, p
-    p = torch.empty(B * H, N, ldp, dtype=qkv.dtype, device=qkv.device)
-    if ldp != N:
-        p[:, :, N:].zero_()
-    q, k, v = qkv[:, :D], qkv[:, D:2 * D], qkv[:, 2 * D:]
-    ld3 = qkv.stride(0)
-    # S = Q K^T  (per (image, head) problem; operands addressed in place inside qkv)
-    gemm_raw(q, ld3, 0, k, ld3, 0, p, ldp, N, N, hd,
-             batch=(H, B, hd, N * ld3, hd, N * ld3, N * ldp, H * N * ldp))
-    _C.softmax_fwd(p, B * H * N, N, ldp, hd ** -0.5)
-    out = torch.empty(B * N, D, dtype=qkv.dtype, device=qkv.device)
+    if kernel == ONESHOT:
+        _C.attention_fwd(qkv, out, None, B, N, H, hd)
+        return out, None
+    p = attention_probs(qkv, B, N, H, hd)
+    pv = p if drop is None else dropout(p, drop[0], drop[1])
+    ldp, ld3 = p.shape[2], qkv.stride(0)
     # O = P V  (V is MN-major: head-dim contiguous, keys strided)
-    gemm_raw(p, ldp, 0, v, ld3, 1, out, D, N, hd, N,
+    gemm_raw(pv, ldp, 0, qkv[:, 2 * D:], ld3, 1, out, D, N, hd, N,
              batch=(H, B, N * ldp, H * N * ldp, hd, N * ld3, hd, N * D))
     return out, p
 
 
-# Fused (flash-style) forward + backward pair: the forward keeps only the row log-sum-exp, the backward kernels
-# (csrc/attention_bwd_sm100.cu) rebuild P tile by tile; scores never reach HBM.  Measured on B200 (CUDA events,
-# profiles/r2_attention.md), forward + backward incl. the P re-materialisation the un-fused path needs:
-#   ViT-L  (B128 N196 H16 hd64) : fused 159 + 387 us   vs un-fused 279 + 500 + 204 us   -> fused by default
-#   336 px (B56 N576 H32 hd160) : fused 1584 + 3032 us vs un-fused 1424 + 2459 + 1088 us, and P alone would be
-#                                 1.2 GB per block                                       -> fused by default
-#   ViT-10B (B128 N256 H32 hd160): fused (persistent, round 2) 311 + 1352 us vs un-fused 664 + 1356 (+426 if P is not
-#                                 kept), and no 512 MiB of P per block                   -> fused by default
-# B200_FUSED_ATTN_BWD=0 / 1 forces the choice.
-_FLASH_ENV = _os.environ.get("B200_FUSED_ATTN_BWD", "")
-FLASH_ATTENTION = _FLASH_ENV != "0"
-FLASH_LONG = _os.environ.get("B200_FUSED_ATTN_LONG", "1") != "0"
-
-
-def flash_supported(N: int, hd: int) -> bool:
-    if N <= 256:
-        return bool(_C.attention_fwd_supported(N, hd) and _C.attention_bwd_supported(N, hd))
-    return bool(FLASH_LONG and _C.attention_fwd_long_supported(N, hd) and _C.attention_bwd_supported(N, hd))
-
-
 def use_flash(N: int, hd: int) -> bool:
     """Model-level policy: run the attention core through the fused forward (log-sum-exp) + fused backward pair?"""
-    if not FLASH_ATTENTION or not flash_supported(N, hd):
-        return False
-    return True
+    return attention_plan.plan(N, hd).fwd_lse is not None
 
 
 def attention_fwd_lse(qkv, B: int, N: int, H: int, hd: int):
+    kernel = attention_plan.plan(N, hd).fwd_lse
     out = torch.empty(B * N, H * hd, dtype=qkv.dtype, device=qkv.device)
     lse = torch.empty(B * H, N, dtype=torch.float32, device=qkv.device)
-    if _persist(hd) and _C.attention_fwd_persist_supported(N, hd):
+    if kernel == PERSIST:
         _C.attention_fwd_persist(qkv, out, lse, B, N, H, hd)
-    elif N <= 256:
-        _C.attention_fwd(qkv, out, lse, None, B, N, H, hd)
-    else:
+    elif kernel == ONESHOT:
+        _C.attention_fwd(qkv, out, lse, B, N, H, hd)
+    elif kernel == LONG:
         _C.attention_fwd_long(qkv, out, lse, B, N, H, hd)
+    else:
+        raise ValueError(f"no fused attention forward for N={N}, hd={hd}")
     return out, lse
 
 
 def attention_bwd_lse(dout, qkv, out, lse, B: int, N: int, H: int, hd: int, want_colsum: bool = False):
+    kernel = attention_plan.plan(N, hd).bwd
+    if kernel not in (ONESHOT, PERSIST):
+        raise ValueError(f"no fused attention backward for N={N}, hd={hd}")
+    persist = kernel == PERSIST
     dqkv = torch.empty(B * N, 3 * H * hd, dtype=qkv.dtype, device=qkv.device)
-    persist = _persist(hd) and N % 4 == 0  # the persistent kernels bulk-copy per-row statistics in 16-byte units
     # scratch: rowsum(dO o O); the persistent kernels get a second plane holding lse * log2(e)
     delta = torch.empty(2 if persist else 1, B * H, N, dtype=torch.float32, device=qkv.device)
     # the persistent kernels reduce the qkv bias gradient (column sums of dq | dk | dv) from their epilogue tiles

@@ -158,10 +158,6 @@ def attention_fwd(qkv, B: int, N: int, H: int, hd: int, drop=None, need_p: bool 
 FLASH_ATTENTION = False
 
 
-def flash_supported(N: int, hd: int) -> bool:
-    return True
-
-
 def use_flash(N: int, hd: int) -> bool:
     return FLASH_ATTENTION
 
